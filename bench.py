@@ -11,11 +11,15 @@ graph launch (b200rl_onpolicy_iterate).
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference-shaped CPU arm (oracle port, all host cores)
     python bench.py --config c3|c5                           # BASELINE configs[2] (Pendulum A2C) / configs[4] (DQN 1M replay), 1 GPU
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed, as DIR/<name>.npy
 
 Prints ONE JSON line (see DESIGN.md "Measurement").  Timing: one CUDA event pair per step on the
 launching stream (L2 flushed between steps, outside the timed region), NO host synchronisation
 inside the loop (the host runs ahead; the intervals are read after the closing barrier),
-barrier + synchronise around the loop, max over ranks."""
+barrier + synchronise around the loop, max over ranks.
+
+Inputs are seeded, so two runs with the same arguments compute from the same inputs; --dump-outputs
+lets two builds be compared output for output.  The benchmark writes nothing into the source tree."""
 import argparse
 import json
 import os
@@ -26,6 +30,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # no __pycache__ in the tree (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -39,6 +44,40 @@ BYTES_K7_SAMPLE = 32             # SURVEY §8d: s 16 + a 4 + logp_old 4 + adv 4 
 BYTES_LOOP_ENV_STEP = 235        # SURVEY §8d: full PPO iteration per env-step (49 + 33 + 25 + 4 x 32)
 METRIC = "env-steps/sec at 65536 CartPole envs (full PPO iteration: rollout T=32 + GAE + 4 epochs x 4 minibatches)"
 PHASE_BASE = 448                 # timer slots used by the per-phase breakdown
+DUMP_MAX_BYTES = 64 << 20        # --dump-outputs: cap on everything written
+DUMP_ENVS = 16384                # --dump-outputs: rollout columns kept (a fixed, seeded sample when there are more envs)
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy, float32 arrays as they are, anything else as float64 (exact for the
+    integer actions, flags and replay keys)."""
+    arrays = {k: np.ascontiguousarray(a, np.float32 if np.asarray(a).dtype == np.float32 else np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte cap")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
+def dump_env_sample(n):
+    """Env columns --dump-outputs keeps: all of them up to DUMP_ENVS, else DUMP_ENVS indices drawn with a fixed seed (sorted)."""
+    if n <= DUMP_ENVS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ENVS, replace=False))
+
+
+def onpolicy_outputs(pkg, agent, net):
+    """What one on-policy iteration hands its caller: the updated parameters, and the rollout it trained on (with values,
+    advantages, returns and the advantage normalisation) for the env columns of dump_env_sample."""
+    R = pkg.learners
+    idx = dump_env_sample(agent.n)
+    out = {"params": net.get(), "adv_norm": agent.rollout(R.ROLL_NORM), "env_index": idx}
+    for name, f in (("state", R.ROLL_STATE), ("action", R.ROLL_ACTION), ("logp", R.ROLL_LOGP), ("reward", R.ROLL_REWARD),
+                    ("terminal", R.ROLL_TERMINAL), ("value", R.ROLL_VALUE), ("advantage", R.ROLL_ADV), ("return", R.ROLL_RET)):
+        a = agent.rollout(f)
+        out[name] = a[:, idx] if f == R.ROLL_STATE else a[idx]
+    return out
 
 
 def measured_peaks():
@@ -390,6 +429,8 @@ def run_c2(args):
     launches0 = ctx.launch_count()
     total_ms = timed_steps(job, lambda: agent.iterate(1), args.steps, sampler)
     launches = ctx.launch_count() - launches0
+    if args.dump_outputs and rank == 0:   # parameters are replicated; the rollout is rank 0's shard
+        write_outputs(args.dump_outputs, onpolicy_outputs(pkg, agent, net))
     clk = sampler.stop() if sampler else None
     graph = agent.graph_active()
     value = n_total * T * args.steps / (total_ms / 1000.0)
@@ -547,6 +588,8 @@ def run_c3(args):
     l0 = ctx.launch_count()
     total_ms = timed_steps(job, lambda: agent.iterate(1), args.steps, sampler)
     launches = ctx.launch_count() - l0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, onpolicy_outputs(pkg, agent, net))
     clk = sampler.stop()
     value = n * T * args.steps / (total_ms / 1000.0)
     ph = phase_breakdown(job, agent, T, 1)
@@ -615,6 +658,10 @@ def run_c5(args):
             learner.update()
     total_ms = timed_steps(job, step, args.steps, sampler)
     launches = ctx.launch_count() - l0
+    if args.dump_outputs:   # the last optimise! call: updated Q-network, the batch it sampled, its TD errors
+        out = {"params": qnet.get(), "td": learner.last_td(), "total_priority": np.array([tr.total_priority()])}
+        out.update(("batch_" + k, a) for k, a in tr.batch().items())
+        write_outputs(args.dump_outputs, out)
     clk = sampler.stop()
     ups = per_step * args.steps / (total_ms / 1000.0)
     # e2e: the user-facing call with the per-update statistics read back to the host (loss, grad norm, mean |td|: a D2H copy + sync per update)
@@ -669,7 +716,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-weak", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float32 / float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (--impl own)")
     if args.impl == "reference":
         run_reference(args)
     elif args.config == "c3":
