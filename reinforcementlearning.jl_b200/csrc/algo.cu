@@ -8,30 +8,10 @@
 // FluxApproximator/optimise! policies/learners/flux_approximator.jl:11-46; TargetNetwork
 // target_network.jl:27-88; PPO/A2C/DQN update rules: ReinforcementLearningZoo (absent from the
 // snapshot; SURVEY Appendix B), hyper-parameters docs/homepage/blog/a_practical_introduction_to_RL.jl/index.html:15238-15286.
+#include "internal.h"
 #include "nn.cuh"
+#include "opt_path.h"
 
-// other translation units
-int b200rl_gae_fused_internal(b200rl_ctx* ctx, float* adv, float* ret, const float* r, const float* v, const uint8_t* term, float gamma,
-                              float lambda, int64_t S, int64_t n_time, double* partials, float* norm2);
-int b200rl_gae_fused_partials_count(int64_t S);
-int b200rl_env_internal_set_traj_targets(b200rl_env* e, void* reward_col, uint8_t* terminal_col);
-int64_t b200rl_env_internal_n(const b200rl_env* e);
-int b200rl_env_internal_kind(const b200rl_env* e);
-int b200rl_env_internal_nobs(const b200rl_env* e);
-b200rl_ctx* b200rl_env_internal_ctx(const b200rl_env* e);
-bool b200rl_env_internal_continuous(const b200rl_env* e);
-struct TrajBatchView { const float* s; const int32_t* a; const float* r; const uint8_t* t; const float* s2; const float* w; int64_t B; int ns; };
-TrajBatchView b200rl_traj_internal_batch(b200rl_traj* t);
-bool b200rl_traj_internal_prioritized(b200rl_traj* t);
-b200rl_ctx* b200rl_traj_internal_ctx(b200rl_traj* t);
-int64_t b200rl_traj_internal_lanes(b200rl_traj* t);
-int b200rl_traj_internal_priority_from_td(b200rl_traj* t, const float* td_dev, float eps, float alpha);
-int b200rl_comm_allreduce_internal(b200rl_ctx* ctx, void* buf, int64_t n, int is_double);
-int b200rl_comm_world(b200rl_ctx* ctx);
-int b200rl_env_internal_kind(const b200rl_env* e);
-int b200rl_env_internal_max_timeout(const b200rl_env* e);
-int b200rl_env_internal_dtype(const b200rl_env* e);
-void b200rl_env_internal_add_steps(b200rl_env* e, uint64_t n);
 static bool fused_rollout_enabled() {   // B200RL_FUSED_ROLLOUT=0: step through plan!/act! launches instead (same results)
     static int v = -1;
     if (v < 0) { const char* e = getenv("B200RL_FUSED_ROLLOUT"); v = (e && e[0] == '0') ? 0 : 1; }
@@ -119,6 +99,69 @@ static int make_descs(const b200rl_net_desc* d, MlpDesc* actor, MlpDesc* critic)
     else REQUIRE(d->n_out >= 1 && d->n_out <= kOutMax, B200RL_ERR_UNSUPPORTED, "n_out must be 1..4");
     *actor = MlpDesc{d->n_in, d->hidden, d->act, d->kind == 1 ? 2 : d->n_out, d->kind == 1 ? 1 : 0};
     *critic = MlpDesc{d->n_in, d->hidden, d->act, 1, 0};
+    return B200RL_OK;
+}
+
+static AcHyper hyper_of(const b200rl_onpolicy_config& c) {
+    return AcHyper{c.clip_range, c.w_actor, c.w_critic, c.w_entropy, c.min_sigma, c.max_sigma, c.normalize_advantage, c.algo};
+}
+
+// rows {4 loss sums, grad norm} (stride 8) -> {actor_loss, critic_loss, entropy, loss, grad_norm, 0} (stride 6), losses = sums * invB
+static void decode_stats_rows(const b200rl_onpolicy_config& c, const float* rows, int n_rows, float invB, float* out) {
+    for (int r = 0; r < n_rows; ++r) {
+        const float* s = rows + (size_t)r * 8;
+        float* o = out + (size_t)r * 6;
+        o[0] = s[0] * invB; o[1] = s[2] * invB; o[2] = s[1] * invB;
+        o[3] = c.w_actor * o[0] + c.w_critic * o[1] - c.w_entropy * o[2];
+        o[4] = s[4]; o[5] = 0.f;
+    }
+}
+
+// Which kernels run the optimiser step of `n` (opt_path.h).  fused: the caller can run the step in the tail of its tensor-core loss +
+// backward launch on a minibatch of B samples.
+static OptPath net_opt_path(const b200rl_net* n, bool fused, const AcHyper& hp, int64_t B) {
+    b200rl_ctx* ctx = n->ctx;
+    P2PTable peers = {};
+    OptPathIn in;
+    in.world = b200rl_comm_world(ctx);
+    in.p2p = b200rl_comm_p2p_table(ctx, &peers);
+    in.exclusive = peers.exclusive != 0;
+    in.fused_step = fused && nn_fused_step_enabled();
+    in.tc_bwd = nn_tc_enabled() && nn_tc_bwd_supported(n->actor, n->critic);
+    in.tail_fits = in.fused_step && in.tc_bwd && nn_tc_fused_tail_fits(ctx, n->actor, hp, B, n->np);
+    in.fits_inbox = (size_t)n->np + 4 <= kP2PXCap;
+    in.coresident = (int)grid_for(n->np, 256) <= ctx->sm_count;
+    return opt_path(in);
+}
+
+// The optimiser state of `n` with the step's hyper-parameters (Cfg: b200rl_onpolicy_config or b200rl_dqn_config).  stats_row (may be
+// null) receives {4 loss sums, grad norm}; tick (may be null) is a device counter the step increments once.
+template <class Cfg>
+static OptStep net_opt_state(const b200rl_net* n, const Cfg& c, float lr, float* stats_row, unsigned int* tick) {
+    OptStep s = {};
+    s.params = n->params; s.grad = n->grad; s.m = n->m; s.v = n->v; s.beta_t = n->beta_t;
+    s.loss_out4 = n->loss4; s.stats_row = stats_row; s.gnorm_out = n->gnorm;
+    s.cta_sumsq = n->cta_sumsq; s.counter = n->counter2; s.tick = tick;
+    s.max_norm = c.max_grad_norm; s.lr = lr; s.b1 = c.beta1; s.b2 = c.beta2; s.eps = c.eps;
+    if (b200rl_comm_p2p_table(n->ctx, &s.tab)) s.seq_ptr = b200rl_comm_p2p_seq_dev(n->ctx);
+    return s;
+}
+
+// The optimiser step on the n_partials gradient rows / n_loss loss rows in n->partial / n->loss_partial, by every path but
+// OPT_FUSED_TAIL (which runs inside the loss + backward launch, nn_ac_loss_grad_step).
+static int net_opt_step(b200rl_net* n, OptPath path, int n_partials, int n_loss, const OptStep& st) {
+    b200rl_ctx* ctx = n->ctx;
+    if (path != OPT_NCCL_CHAIN) return nn_reduce_clip_adam(ctx, n->partial, n_partials, n->np, n->loss_partial, n_loss, st);
+    TRY(nn_reduce_partials(ctx, n->partial, n_partials, n->np, st.grad, n->loss_partial, n_loss, st.loss_out4));
+    if (b200rl_comm_world(ctx) > 1) {
+        TRY(b200rl_comm_allreduce_internal(ctx, st.grad, n->np, 0));
+        TRY(b200rl_comm_allreduce_internal(ctx, st.loss_out4, 4, 0));
+    }
+    TRY(nn_clip_adam(ctx, st.params, st.grad, st.m, st.v, st.beta_t, n->np, st.max_norm, st.lr, st.b1, st.b2, st.eps, 1.0f, st.gnorm_out));
+    if (st.stats_row) {
+        stats_row_kernel<<<1, 32, 0, ctx->stream>>>(st.stats_row, st.loss_out4, st.gnorm_out, st.tick);
+        LAUNCH_CHECK(ctx);
+    }
     return B200RL_OK;
 }
 
@@ -360,7 +403,7 @@ int b200rl_net_ac_step(b200rl_net* n, const b200rl_onpolicy_config* cfg, const f
     float nm[2] = {adv_mean, adv_inv_std};
     CUDA_TRY(cudaMemcpyAsync(base + o_n, nm, 8, cudaMemcpyHostToDevice, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));  // host buffers (incl. the local iota) are borrowed for this call only
-    AcHyper hp{cfg->clip_range, cfg->w_actor, cfg->w_critic, cfg->w_entropy, cfg->min_sigma, cfg->max_sigma, cfg->normalize_advantage, cfg->algo};
+    const AcHyper hp = hyper_of(*cfg);
     AcBatch b{(const float*)(base + o_s), ns, base + o_a, logp_old ? (const float*)(base + o_l) : nullptr, (const float*)(base + o_ad),
               (const float*)(base + o_r), (const int32_t*)(base + o_i), (uint32_t)total, 0u, 0u, nullptr, nullptr, Beff, 1.0f / (float)Beff,
               (const float*)(base + o_n)};
@@ -372,14 +415,11 @@ int b200rl_net_ac_step(b200rl_net* n, const b200rl_onpolicy_config* cfg, const f
         n->n_updates += 1;
     }
     if (losses_out) {
-        float l4[4], gn = 0.f;
-        CUDA_TRY(cudaMemcpyAsync(l4, n->loss4, 16, cudaMemcpyDeviceToHost, ctx->stream));
-        if (apply_update) CUDA_TRY(cudaMemcpyAsync(&gn, n->gnorm, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        float row[8] = {};   // {4 loss sums, grad norm}
+        CUDA_TRY(cudaMemcpyAsync(row, n->loss4, 16, cudaMemcpyDeviceToHost, ctx->stream));
+        if (apply_update) CUDA_TRY(cudaMemcpyAsync(row + 4, n->gnorm, 4, cudaMemcpyDeviceToHost, ctx->stream));
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        float invB = 1.0f / (float)Beff;
-        losses_out[0] = l4[0] * invB; losses_out[1] = l4[2] * invB; losses_out[2] = l4[1] * invB;
-        losses_out[3] = cfg->w_actor * losses_out[0] + cfg->w_critic * losses_out[1] - cfg->w_entropy * losses_out[2];
-        losses_out[4] = gn; losses_out[5] = 0.f;
+        decode_stats_rows(*cfg, row, 1, 1.0f / (float)Beff, losses_out);
     }
     return B200RL_OK;
 }
@@ -410,6 +450,17 @@ struct b200rl_onpolicy {
 };
 
 static void* env_field(b200rl_env* e, int f) { void* p = nullptr; b200rl_env_ptr(e, f, &p); return p; }
+
+static int64_t minibatch_size(const b200rl_onpolicy* a) { return a->N * a->T / a->cfg.n_microbatches; }   // per rank
+static OptPath onpolicy_opt_path(const b200rl_onpolicy* a) { return net_opt_path(a->net, true, hyper_of(a->cfg), minibatch_size(a)); }
+// the stats rows of the last update -> stats_host (n_epochs * n_microbatches, 6)
+static int onpolicy_read_stats(b200rl_onpolicy* a, float* stats_host) {
+    std::vector<float> tmp((size_t)a->stats_rows * 8);
+    CUDA_TRY(cudaMemcpyAsync(tmp.data(), a->stats_dev, tmp.size() * 4, cudaMemcpyDeviceToHost, a->ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(a->ctx->stream));
+    decode_stats_rows(a->cfg, tmp.data(), a->stats_rows, 1.0f / ((float)minibatch_size(a) * (float)b200rl_comm_world(a->ctx)), stats_host);
+    return B200RL_OK;
+}
 
 extern "C" {
 
@@ -485,8 +536,7 @@ int b200rl_onpolicy_plan(b200rl_onpolicy* a, void* actions_host) {
     a->bootstrap_done = false;
     int64_t N = a->N;
     const float* obs = (const float*)env_field(a->env, B200RL_FIELD_OBS);
-    AcHyper hp{a->cfg.clip_range, a->cfg.w_actor, a->cfg.w_critic, a->cfg.w_entropy, a->cfg.min_sigma, a->cfg.max_sigma,
-               a->cfg.normalize_advantage, a->cfg.algo};
+    const AcHyper hp = hyper_of(a->cfg);
     char* act_col = (char*)a->actions + (size_t)N * a->t * 4;
     TRY(nn_policy_act(a->ctx, a->net->actor, a->net->critic, a->net->params, hp, obs, N, a->rng, act_col, a->logp + (size_t)N * a->t,
                       a->values + (size_t)N * a->t, nullptr, a->states + (size_t)N * a->ns * a->t));
@@ -524,8 +574,7 @@ int b200rl_onpolicy_collect(b200rl_onpolicy* a, int n_steps) {
     if (n_steps > 0 && nn_tc_enabled() && fused_rollout_enabled()) {   // one launch for the whole stretch (fwd_tc.cu)
         REQUIRE(a->t + n_steps <= a->T, B200RL_ERR_INVALID, "rollout is full: call b200rl_onpolicy_update first");
         TRY(ctx_bind(a->ctx));
-        AcHyper hp{a->cfg.clip_range, a->cfg.w_actor, a->cfg.w_critic, a->cfg.w_entropy, a->cfg.min_sigma, a->cfg.max_sigma,
-                   a->cfg.normalize_advantage, a->cfg.algo};
+        const AcHyper hp = hyper_of(a->cfg);
         const int fin = a->t + n_steps == a->T ? 1 : 0;
         int st = nn_tc_rollout(a->ctx, a->env, a->net->actor, a->net->critic, a->net->params, hp, a->rng, a->t, n_steps, a->T, fin, a->states,
                                a->actions, a->logp, a->values, a->rewards, a->terminals);
@@ -608,8 +657,9 @@ int b200rl_onpolicy_update(b200rl_onpolicy* a, const int32_t* perm_host, float* 
         CUDA_TRY(cudaMemcpyAsync(a->perm_dev, perm_host, (size_t)c.n_epochs * NT_ * 4, cudaMemcpyHostToDevice, ctx->stream));
     }
     TRY(phase(1));
-    AcHyper hp{c.clip_range, c.w_actor, c.w_critic, c.w_entropy, c.min_sigma, c.max_sigma, c.normalize_advantage, c.algo};
-    int64_t B = NT_ / c.n_microbatches;
+    const AcHyper hp = hyper_of(c);
+    const int64_t B = minibatch_size(a);
+    const OptPath path = onpolicy_opt_path(a);
     int row = 0;
     for (int e = 0; e < c.n_epochs; ++e) {
         for (int mb = 0; mb < c.n_microbatches; ++mb, ++row) {
@@ -621,30 +671,16 @@ int b200rl_onpolicy_update(b200rl_onpolicy* a, const int32_t* perm_host, float* 
                       1.0f / ((float)B * (float)world), a->norm2};
             float* stats_row = a->stats_dev + (size_t)row * 8;
             unsigned int* tick = row == a->stats_rows - 1 ? a->upd_dev : nullptr;   // the last optimiser step closes the update
-            // one launch: loss + backward + [peer exchange] + clip + Adam (tensor-core path)
-            int ctas = nn_ac_loss_grad_step(ctx, n->actor, n->critic, n->params, hp, b, n->partial, n->loss_partial, n->grad, n->m, n->v, n->beta_t,
-                                            n->loss4, c.max_grad_norm, c.lr, c.beta1, c.beta2, c.eps, n->gnorm, n->cta_sumsq, n->counter2, stats_row, tick);
-            if (ctas > 0) {
+            const OptStep st = net_opt_state(n, c, c.lr, stats_row, tick);
+            if (path == OPT_FUSED_TAIL) {   // one launch: loss + backward + [peer exchange] + clip + Adam
+                const int ctas = nn_ac_loss_grad_step(ctx, n->actor, n->critic, hp, b, n->partial, n->loss_partial, st);
+                if (ctas < 0) return ctas;
                 TRY(phase(2 + 2 * row));
-                TRY(phase(3 + 2 * row));
-                n->n_updates += 1;
-                continue;
-            }
-            if (ctas != B200RL_ERR_UNSUPPORTED) return ctas;
-            ctas = nn_ac_loss_grad(ctx, n->actor, n->critic, n->params, hp, b, n->partial, n->loss_partial);
-            if (ctas < 0) return ctas;
-            TRY(phase(2 + 2 * row));
-            P2PTable peers;
-            if (world > 1 && !b200rl_comm_p2p_table(ctx, &peers)) {   // no peer exchange attached: reduce -> NCCL all-reduce -> clip + Adam
-                TRY(nn_reduce_partials(ctx, n->partial, ctas, n->np, n->grad, n->loss_partial, 2 * ctas, n->loss4));
-                TRY(b200rl_comm_allreduce_internal(ctx, n->grad, n->np, 0));
-                TRY(b200rl_comm_allreduce_internal(ctx, n->loss4, 4, 0));
-                TRY(nn_clip_adam(ctx, n->params, n->grad, n->m, n->v, n->beta_t, n->np, c.max_grad_norm, c.lr, c.beta1, c.beta2, c.eps, 1.0f, n->gnorm));
-                stats_row_kernel<<<1, 32, 0, ctx->stream>>>(stats_row, n->loss4, n->gnorm, tick);
-                LAUNCH_CHECK(ctx);
-            } else {   // one kernel: reduce [-> exchange with the peers over NVLink] -> clip -> Adam -> stats row
-                TRY(nn_reduce_clip_adam(ctx, n->partial, ctas, n->np, n->params, n->grad, n->m, n->v, n->beta_t, n->loss_partial, 2 * ctas, n->loss4,
-                                        c.max_grad_norm, c.lr, c.beta1, c.beta2, c.eps, n->gnorm, n->cta_sumsq, n->counter2, stats_row, tick));
+            } else {
+                const int ctas = nn_ac_loss_grad(ctx, n->actor, n->critic, n->params, hp, b, n->partial, n->loss_partial);
+                if (ctas < 0) return ctas;
+                TRY(phase(2 + 2 * row));
+                TRY(net_opt_step(n, path, ctas, 2 * ctas, st));
             }
             TRY(phase(3 + 2 * row));
             n->n_updates += 1;
@@ -652,19 +688,7 @@ int b200rl_onpolicy_update(b200rl_onpolicy* a, const int32_t* perm_host, float* 
     }
     a->n_updates += 1;
     a->t = 0;
-    if (stats_host) {
-        std::vector<float> tmp((size_t)a->stats_rows * 8);
-        CUDA_TRY(cudaMemcpyAsync(tmp.data(), a->stats_dev, tmp.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        float invB = 1.0f / ((float)B * (float)world);
-        for (int r = 0; r < a->stats_rows; ++r) {
-            float* o = stats_host + (size_t)r * 6;
-            const float* s = tmp.data() + (size_t)r * 8;
-            o[0] = s[0] * invB; o[1] = s[2] * invB; o[2] = s[1] * invB;
-            o[3] = c.w_actor * o[0] + c.w_critic * o[1] - c.w_entropy * o[2];
-            o[4] = s[4]; o[5] = 0.f;
-        }
-    }
+    if (stats_host) TRY(onpolicy_read_stats(a, stats_host));
     return B200RL_OK;
 }
 
@@ -683,8 +707,7 @@ int b200rl_onpolicy_iterate(b200rl_onpolicy* a, int n_iters, float* stats_host) 
     b200rl_ctx* ctx = a->ctx;
     static int graph_env = -1;
     if (graph_env < 0) { const char* e = getenv("B200RL_GRAPH"); graph_env = (e && e[0] == '0') ? 0 : 1; }
-    P2PTable peers;
-    const bool capturable = graph_env && !a->graph_failed && ctx->phase_base < 0 && (b200rl_comm_world(ctx) == 1 || b200rl_comm_p2p_table(ctx, &peers));
+    const bool capturable = graph_env && !a->graph_failed && ctx->phase_base < 0 && onpolicy_opt_path(a) != OPT_NCCL_CHAIN;
     const int rows = a->stats_rows;
     for (int it = 0; it < n_iters; ++it) {
         if (!capturable || !a->warmed) {
@@ -734,20 +757,7 @@ int b200rl_onpolicy_iterate(b200rl_onpolicy* a, int n_iters, float* stats_host) 
         a->n_updates += 1; a->net->n_updates += (uint64_t)rows;
         b200rl_env_internal_add_steps(a->env, (uint64_t)a->T);
     }
-    if (stats_host && n_iters > 0) {
-        const b200rl_onpolicy_config& c = a->cfg;
-        std::vector<float> tmp((size_t)rows * 8);
-        CUDA_TRY(cudaMemcpyAsync(tmp.data(), a->stats_dev, tmp.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        float invB = 1.0f / ((float)(a->N * a->T / c.n_microbatches) * (float)b200rl_comm_world(ctx));
-        for (int r = 0; r < rows; ++r) {
-            float* o = stats_host + (size_t)r * 6;
-            const float* s = tmp.data() + (size_t)r * 8;
-            o[0] = s[0] * invB; o[1] = s[2] * invB; o[2] = s[1] * invB;
-            o[3] = c.w_actor * o[0] + c.w_critic * o[1] - c.w_entropy * o[2];
-            o[4] = s[4]; o[5] = 0.f;
-        }
-    }
+    if (stats_host && n_iters > 0) TRY(onpolicy_read_stats(a, stats_host));
     return B200RL_OK;
 }
 /* 1 when b200rl_onpolicy_iterate replays a captured graph, 0 when it launches eagerly (diagnostic for tests / bench) */
@@ -836,9 +846,9 @@ int b200rl_onpolicy_time_kernel(b200rl_onpolicy* a, int which, int reps, float* 
     b200rl_net* n = a->net;
     const b200rl_onpolicy_config& c = a->cfg;
     int64_t N = a->N, T = a->T, NT_ = N * T, B = NT_ / c.n_microbatches;
-    AcHyper hp{c.clip_range, c.w_actor, c.w_critic, c.w_entropy, c.min_sigma, c.max_sigma, c.normalize_advantage, c.algo};
+    const AcHyper hp = hyper_of(c);
     const float* obs = (const float*)env_field(a->env, B200RL_FIELD_OBS);
-    int ctas = (nn_tc_enabled() && nn_tc_bwd_supported(n->actor, n->critic)) ? nn_tc_partial_rows(2 * (ctx->sm_count / 2), n->actor, hp, B) : nn_grid_ctas(ctx, n->actor.H);
+    const int ctas = nn_ac_partial_rows(ctx, n->actor, n->critic, hp, B);
     void* rng_copy = nullptr;
     if (which == 1) {
         TRY(ctx_scratch(ctx, (size_t)N * 32 + (size_t)N * 12 + 256, &rng_copy));
@@ -858,17 +868,8 @@ int b200rl_onpolicy_time_kernel(b200rl_onpolicy* a, int which, int reps, float* 
             }
             case 2: return b200rl_env_step(a->env, a->actions, 1, 1);
             case 3: return b200rl_gae_fused_internal(ctx, a->adv, a->ret, a->rewards, a->values, a->terminals, c.gamma, c.lambda, N, T, a->norm_partials, nullptr);
-            case 4: {   // the optimiser step as update() runs it (lr = 0: parameters stay put), incl. the peer exchange of a sharded run
-                P2PTable peers;
-                if (b200rl_comm_world(ctx) > 1 && !b200rl_comm_p2p_table(ctx, &peers)) {
-                    TRY(nn_reduce_partials(ctx, n->partial, ctas, n->np, n->grad, n->loss_partial, 2 * ctas, n->loss4));
-                    TRY(b200rl_comm_allreduce_internal(ctx, n->grad, n->np, 0));
-                    TRY(b200rl_comm_allreduce_internal(ctx, n->loss4, 4, 0));
-                    return nn_clip_adam(ctx, n->params, n->grad, n->m, n->v, n->beta_t, n->np, c.max_grad_norm, 0.0f, c.beta1, c.beta2, c.eps, 1.0f, n->gnorm);
-                }
-                return nn_reduce_clip_adam(ctx, n->partial, ctas, n->np, n->params, n->grad, n->m, n->v, n->beta_t, n->loss_partial, 2 * ctas, n->loss4,
-                                           c.max_grad_norm, 0.0f, c.beta1, c.beta2, c.eps, n->gnorm, n->cta_sumsq, n->counter2, nullptr, nullptr);
-            }
+            case 4:   // the unfused optimiser step as update() runs it (lr = 0: parameters stay put), incl. the exchange of a sharded run
+                return net_opt_step(n, net_opt_path(n, false, hp, B), ctas, 2 * ctas, net_opt_state(n, c, 0.0f, nullptr, nullptr));
         }
         b200rl_set_error("unknown kernel id");
         return B200RL_ERR_INVALID;
@@ -919,20 +920,7 @@ int b200rl_dqn_update(b200rl_net* n, b200rl_traj* t, const b200rl_dqn_config* cf
     int np_ = nn_dqn_loss_grad(ctx, n->actor, n->params, n->target, b.s, b.a, b.r, b.t, b.s2, b.w, b.B, 1.0f / ((float)b.B * (float)world), cfg->gamma,
                                cfg->huber, cfg->double_dqn, n->partial, n->loss_partial, td);
     if (np_ < 0) return np_;
-    P2PTable peers;
-    const unsigned adam_grid = grid_for(n->np, 256);
-    if ((world == 1 || b200rl_comm_p2p_table(ctx, &peers)) && (int)adam_grid <= ctx->sm_count) {
-        // one kernel: partial reduce [-> peer exchange] -> global-norm clip -> Adam (the optimiser step of the on-policy path)
-        TRY(nn_reduce_clip_adam(ctx, n->partial, np_, n->np, n->params, n->grad, n->m, n->v, n->beta_t, n->loss_partial, np_, n->loss4, cfg->max_grad_norm,
-                                cfg->lr, cfg->beta1, cfg->beta2, cfg->eps, n->gnorm, n->cta_sumsq, n->counter2, nullptr, nullptr));
-    } else {
-        TRY(nn_reduce_partials(ctx, n->partial, np_, n->np, n->grad, n->loss_partial, np_, n->loss4));
-        if (world > 1) {
-            TRY(b200rl_comm_allreduce_internal(ctx, n->grad, n->np, 0));
-            TRY(b200rl_comm_allreduce_internal(ctx, n->loss4, 4, 0));
-        }
-        TRY(nn_clip_adam(ctx, n->params, n->grad, n->m, n->v, n->beta_t, n->np, cfg->max_grad_norm, cfg->lr, cfg->beta1, cfg->beta2, cfg->eps, 1.0f, n->gnorm));
-    }
+    TRY(net_opt_step(n, net_opt_path(n, false, AcHyper{}, b.B), np_, np_, net_opt_state(n, *cfg, cfg->lr, nullptr, nullptr)));
     if (b200rl_traj_internal_prioritized(t)) TRY(b200rl_traj_internal_priority_from_td(t, td, cfg->per_eps, cfg->per_alpha));
     n->n_updates += 1;
     if (cfg->target_update_freq > 0 && n->n_updates % (uint64_t)cfg->target_update_freq == 0) TRY(nn_target_sync(ctx, n->target, n->params, n->np, cfg->rho));

@@ -5,7 +5,7 @@
 // link-time dependency and shares the NCCL already loaded by the host process (e.g. torch's).
 #include <dlfcn.h>
 
-#include "common.cuh"
+#include "internal.h"
 
 namespace {
 typedef struct ncclComm* ncclComm_t;

@@ -2,7 +2,7 @@
 #include <cstdarg>
 #include <cstdlib>
 
-#include "common.cuh"
+#include "internal.h"
 
 static thread_local char g_err[1024] = "no error";
 
@@ -33,8 +33,6 @@ __global__ void flush_kernel(float4* p, size_t n) {
     size_t stride = (size_t)gridDim.x * blockDim.x;
     for (; i < n; i += stride) p[i] = make_float4(1.f, 2.f, 3.f, 4.f);
 }
-
-void b200rl_comm_destroy_internal(b200rl_ctx* ctx);
 
 extern "C" {
 

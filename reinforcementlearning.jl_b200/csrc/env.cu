@@ -13,6 +13,7 @@
 
 #include "common.cuh"
 #include "env_device.cuh"
+#include "internal.h"
 
 using jld::Xo;
 using namespace envdev;

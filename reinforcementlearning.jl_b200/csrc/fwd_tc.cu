@@ -10,13 +10,11 @@
 // (-fmad=false): stepping through plan!/act! one launch at a time or through the fused rollout gives bit-identical results.
 #include "common.cuh"
 #include "env_device.cuh"
+#include "internal.h"
 #include "tc_fwd.cuh"
 
 using namespace tcfwd;
 using namespace envdev;
-
-int b200rl_env_internal_view(b200rl_env* e, envdev::EnvView* out);
-void b200rl_env_internal_add_steps(b200rl_env* e, uint64_t n);
 
 namespace {
 

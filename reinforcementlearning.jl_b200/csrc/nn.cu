@@ -13,7 +13,8 @@
 // (RLCore/src/utils/networks.jl:405-432), Gaussian head + diagnormlogpdf (networks.jl:44-116,
 // distributions.jl:9-34), clip_by_global_norm! (basic.jl:19-29), TargetNetwork sync
 // (policies/learners/target_network.jl:70-88).
-#include "nn.cuh"
+#include "opt_path.h"
+#include "optim.cuh"
 #include "perm.cuh"
 
 namespace {
@@ -711,9 +712,7 @@ __global__ void __launch_bounds__(1024) clip_adam_kernel(float* __restrict__ p, 
         double t = 0.0;
         for (int k = 0; k < (int)(blockDim.x >> 5); ++k) t += red[k];
         float gn = (float)sqrt(t);
-        float sc = 1.0f;
-        if (max_norm > 0.f && max_norm <= gn) sc = max_norm / fmaxf(max_norm, gn);
-        s_scale = sc;
+        s_scale = clip_scale(gn, max_norm);
         if (gnorm_out) *gnorm_out = gn;
     }
     __syncthreads();
@@ -722,10 +721,7 @@ __global__ void __launch_bounds__(1024) clip_adam_kernel(float* __restrict__ p, 
     for (int64_t k = threadIdx.x; k < np; k += blockDim.x) {
         float gk = g[k] * sc;
         g[k] = gk;
-        float mk = b1 * m[k] + (1.0f - b1) * gk;
-        float vk = b2 * v[k] + (1.0f - b2) * (gk * gk);
-        m[k] = mk; v[k] = vk;
-        p[k] -= mk / (1.0f - bt1) / (sqrtf(vk / (1.0f - bt2)) + eps) * lr;
+        p[k] -= adam_apply(gk, m[k], v[k], b1, b2, eps, lr, bt1, bt2);
     }
     __syncthreads();
     if (threadIdx.x == 0) { beta_t[0] = bt1 * b1; beta_t[1] = bt2 * b2; }
@@ -738,20 +734,17 @@ __global__ void __launch_bounds__(1024) clip_adam_kernel(float* __restrict__ p, 
 // self-validating {value, sequence} packet (remote NVLink store), then reads the peers' packets from the own inbox and sums
 // in rank order — every rank computes the identical global gradient, so the replicas stay bit-identical without a broadcast.
 template <bool XCHG>
-__global__ void __launch_bounds__(256) reduce_clip_adam_kernel(const float* __restrict__ partial, int n_partials, int64_t np, float* __restrict__ p,
-                                                              float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
-                                                              float* __restrict__ beta_t, const float* __restrict__ loss_partial, int n_loss,
-                                                              float* __restrict__ loss_out4, float max_norm, float lr, float b1, float b2, float eps,
-                                                              float* __restrict__ gnorm_out, double* __restrict__ cta_sumsq,
-                                                              unsigned int* __restrict__ counter, float* __restrict__ stats_row,
-                                                              P2PTable tab, unsigned int* __restrict__ seq_ptr, unsigned int* __restrict__ tick) {
+__global__ void __launch_bounds__(256) reduce_clip_adam_kernel(const float* __restrict__ partial, int n_partials, int64_t np,
+                                                              const float* __restrict__ loss_partial, int n_loss, OptStep st) {
     __shared__ double red[8];
     __shared__ float s_scale;
     // The grid barrier counters reset themselves (the last CTA through the second counter zeroes both), the exchange sequence
     // number and the update tick live in device memory: nothing here depends on host-side launch counts, so the launch can be
     // captured in a CUDA graph and replayed, and no counter ever wraps.
+    float* __restrict__ p = st.params; float* __restrict__ g = st.grad; float* __restrict__ m = st.m; float* __restrict__ v = st.v;
+    const P2PTable& tab = st.tab;
     const unsigned int target = gridDim.x;
-    const unsigned int seq = XCHG ? *seq_ptr + 1u : 0u;
+    const unsigned int seq = XCHG ? *st.seq_ptr + 1u : 0u;
     const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     float gk = 0.f;
     if (k < np) {
@@ -765,16 +758,12 @@ __global__ void __launch_bounds__(256) reduce_clip_adam_kernel(const float* __re
         const unsigned slot = seq & 1u;
         if (k < np) p2p_push(tab, 0, slot, (size_t)k, __float_as_uint(gk), seq);
         if (loss_thread) p2p_push(tab, 0, slot, (size_t)np + threadIdx.x, __float_as_uint(lsum), seq);   // the 4 loss sums ride along
-        float acc = 0.f, lacc = 0.f;
-        for (int r = 0; r < tab.nranks; ++r) {
-            if (k < np) acc += r == tab.rank ? gk : __uint_as_float(p2p_recv(tab, 0, slot, r, (size_t)k, seq));
-            if (loss_thread) lacc += r == tab.rank ? lsum : __uint_as_float(p2p_recv(tab, 0, slot, r, (size_t)np + threadIdx.x, seq));
-        }
-        gk = acc; lsum = lacc;
+        if (k < np) gk = p2p_sum_rank_order(tab, slot, (size_t)k, gk, seq);
+        if (loss_thread) lsum = p2p_sum_rank_order(tab, slot, (size_t)np + threadIdx.x, lsum, seq);
     }
     if (loss_thread) {
-        if (loss_out4) loss_out4[threadIdx.x] = lsum;
-        if (stats_row) stats_row[threadIdx.x] = lsum;
+        if (st.loss_out4) st.loss_out4[threadIdx.x] = lsum;
+        if (st.stats_row) st.stats_row[threadIdx.x] = lsum;
     }
     double acc = (double)gk * (double)gk;
 #pragma unroll
@@ -785,54 +774,39 @@ __global__ void __launch_bounds__(256) reduce_clip_adam_kernel(const float* __re
         if (threadIdx.x == 0) {
             double t = 0.0;
             for (int w = 0; w < 8; ++w) t += red[w];
-            cta_sumsq[blockIdx.x] = t;
-            __threadfence();
-            atomicAdd(counter, 1u);
-            unsigned int spins = 0;
-            while (*reinterpret_cast<volatile unsigned int*>(counter) < target)
-                if (++spins > (1u << 26)) __trap();
-            __threadfence();
+            st.cta_sumsq[blockIdx.x] = t;
+            grid_arrive_wait(st.counter, target);
         }
         __syncwarp();
         // (one dependent L2 read per CTA was ~5 us of this ~14 us kernel; the loads now go out together, the adds keep the CTA order)
         double tot = 0.0;
         for (unsigned int c0 = 0; c0 < gridDim.x; c0 += 32) {
             const unsigned int c = c0 + threadIdx.x;
-            const double mine = c < gridDim.x ? *reinterpret_cast<volatile double*>(cta_sumsq + c) : 0.0;
+            const double mine = c < gridDim.x ? *reinterpret_cast<volatile double*>(st.cta_sumsq + c) : 0.0;
             const unsigned int n = min(32u, gridDim.x - c0);
             for (unsigned int l = 0; l < n; ++l) tot += __shfl_sync(0xffffffffu, mine, l);
         }
     if (threadIdx.x == 0) {
         float gn = (float)sqrt(tot);
-        float sc = 1.0f;
-        if (max_norm > 0.f && max_norm <= gn) sc = max_norm / fmaxf(max_norm, gn);
-        s_scale = sc;
+        s_scale = clip_scale(gn, st.max_norm);
         if (blockIdx.x == 0) {
-            if (gnorm_out) *gnorm_out = gn;
-            if (stats_row) stats_row[4] = gn;
+            if (st.gnorm_out) *st.gnorm_out = gn;
+            if (st.stats_row) st.stats_row[4] = gn;
         }
     }
     }
     __syncthreads();
-    const float bt1 = beta_t[0], bt2 = beta_t[1];
+    const float bt1 = st.beta_t[0], bt2 = st.beta_t[1];
     if (k < np) {
         gk *= s_scale;
         g[k] = gk;
-        float mk = b1 * m[k] + (1.0f - b1) * gk;
-        float vk = b2 * v[k] + (1.0f - b2) * (gk * gk);
-        m[k] = mk; v[k] = vk;
-        p[k] -= mk / (1.0f - bt1) / (sqrtf(vk / (1.0f - bt2)) + eps) * lr;
+        p[k] -= adam_apply(gk, m[k], v[k], st.b1, st.b2, st.eps, st.lr, bt1, bt2);
     }
     // beta^t advances once every CTA has read it: the last CTA to pass a second counter does it
     __syncthreads();
     if (threadIdx.x == 0) {
         __threadfence();
-        if (atomicAdd(counter + 1, 1u) + 1u == target) {   // every CTA has left the first barrier and read beta^t / the sequence number
-            beta_t[0] = bt1 * b1; beta_t[1] = bt2 * b2;
-            counter[0] = 0u; counter[1] = 0u;
-            if (XCHG) *seq_ptr = seq;
-            if (tick) *tick += 1u;
-        }
+        last_cta_epilogue(st, st.counter + 1, 2, target, bt1, bt2, XCHG, seq);
     }
 }
 
@@ -1024,6 +998,11 @@ bool nn_tc_enabled() {
 extern "C" int b200rl_set_tensor_cores(int enable) { g_tc = enable ? 1 : 0; return B200RL_OK; }
 static int g_fused_step = -1;   // -1: not decided yet (environment), see nn_ac_loss_grad_step
 extern "C" int b200rl_set_fused_step(int enable) { g_fused_step = enable ? 1 : 0; return B200RL_OK; }
+bool nn_fused_step_enabled() {
+    if (g_fused_step < 0) { const char* e = getenv("B200RL_FUSED_STEP"); g_fused_step = (e && e[0] == '0') ? 0 : 1; }
+    return g_fused_step != 0;
+}
+static int tc_grid(b200rl_ctx* ctx) { return 2 * (ctx->sm_count / 2); }   // one 512-thread CTA per SM, split between the roles (nn_tc_actor_ctas)
 
 int nn_grid_ctas(b200rl_ctx* ctx, int H) { return H == 64 ? ctx->sm_count : ctx->sm_count / 2; }
 
@@ -1099,43 +1078,32 @@ int nn_ac_loss_grad(b200rl_ctx* ctx, const MlpDesc& actor, const MlpDesc& critic
                     float* partial, float* loss_partial) {
     TRY(check_desc(actor)); TRY(check_desc(critic));
     REQUIRE(actor.H == critic.H && actor.in == critic.in, B200RL_ERR_UNSUPPORTED, "actor and critic must share widths");
-    int ctas = nn_grid_ctas(ctx, actor.H);
     int64_t np = actor.nparams() + critic.nparams();
     int st;
-    if (nn_tc_enabled() && nn_tc_bwd_supported(actor, critic)) {
-        const int grid = 2 * (ctx->sm_count / 2);   // one 512-thread CTA per SM, split between the roles (nn_tc_actor_ctas)
-        ctas = nn_tc_partial_rows(grid, actor, hp, b.B);
-        st = nn_tc_ac_loss_grad(ctx, grid, actor, critic, params, hp, b, partial, loss_partial, np, nullptr);
-    } else if (actor.H == 64) {
-        st = launch_ac<64>(ctx, 2 * ctas, actor, critic, params, hp, b, partial, loss_partial, np);
-    } else {
-        st = launch_ac<128>(ctx, 2 * ctas, actor, critic, params, hp, b, partial, loss_partial, np);
-    }
-    return st != B200RL_OK ? st : ctas;  // number of gradient partials written (loss rows = 2x)
+    if (nn_tc_enabled() && nn_tc_bwd_supported(actor, critic))
+        st = nn_tc_ac_loss_grad(ctx, tc_grid(ctx), actor, critic, params, hp, b, partial, loss_partial, np, nullptr);
+    else if (actor.H == 64)
+        st = launch_ac<64>(ctx, 2 * nn_grid_ctas(ctx, 64), actor, critic, params, hp, b, partial, loss_partial, np);
+    else
+        st = launch_ac<128>(ctx, 2 * nn_grid_ctas(ctx, 128), actor, critic, params, hp, b, partial, loss_partial, np);
+    return st != B200RL_OK ? st : nn_ac_partial_rows(ctx, actor, critic, hp, b.B);  // number of gradient partials written (loss rows = 2x)
+}
+int nn_ac_partial_rows(b200rl_ctx* ctx, const MlpDesc& actor, const MlpDesc& critic, const AcHyper& hp, int64_t B) {
+    if (nn_tc_enabled() && nn_tc_bwd_supported(actor, critic)) return nn_tc_partial_rows(tc_grid(ctx), actor, hp, B);
+    return nn_grid_ctas(ctx, actor.H);
+}
+bool nn_tc_fused_tail_fits(b200rl_ctx* ctx, const MlpDesc& actor, const AcHyper& hp, int64_t B, int64_t np) {
+    return opt_fused_tail_fits(np, tc_grid(ctx), nn_tc_partial_rows(tc_grid(ctx), actor, hp, B), ctx->sm_count);
 }
 
-// K7 + optimiser step in ONE launch (tensor-core path only; B200RL_FUSED_STEP=0 disables it).  A sharded run takes it only when
-// every rank owns its device (P2PTable::exclusive): the launch occupies all SMs and waits for the peers' packets inside itself.
-int nn_ac_loss_grad_step(b200rl_ctx* ctx, const MlpDesc& actor, const MlpDesc& critic, float* params, const AcHyper& hp, const AcBatch& b,
-                         float* partial, float* loss_partial, float* grad, float* m, float* v, float* beta_t, float* loss_out4,
-                         float max_grad_norm, float lr, float b1, float b2, float eps, float* gnorm_out, double* cta_sumsq,
-                         unsigned int* counter4, float* stats_row, unsigned int* tick) {
-    if (g_fused_step < 0) { const char* e = getenv("B200RL_FUSED_STEP"); g_fused_step = (e && e[0] == '0') ? 0 : 1; }
-    if (!g_fused_step || !nn_tc_enabled() || !nn_tc_bwd_supported(actor, critic) || actor.H != critic.H || actor.in != critic.in) return B200RL_ERR_UNSUPPORTED;
-    if (check_desc(actor) != B200RL_OK || check_desc(critic) != B200RL_OK) return B200RL_ERR_UNSUPPORTED;
-    const int ctas = ctx->sm_count / 2;
+// K7 + optimiser step in ONE launch.  A sharded run takes it only when every rank owns its device (P2PTable::exclusive): the launch
+// occupies all SMs and waits for the peers' packets inside itself.
+int nn_ac_loss_grad_step(b200rl_ctx* ctx, const MlpDesc& actor, const MlpDesc& critic, const AcHyper& hp, const AcBatch& b, float* partial,
+                         float* loss_partial, const OptStep& st) {
+    TRY(check_desc(actor)); TRY(check_desc(critic));
     const int64_t np = actor.nparams() + critic.nparams();
-    if ((np + 2 * ctas - 1) / (2 * ctas) > 512) return B200RL_ERR_UNSUPPORTED;
-    AcStep st = {};
-    st.params = params; st.grad = grad; st.m = m; st.v = v; st.beta_t = beta_t; st.loss_out4 = loss_out4; st.stats_row = stats_row;
-    st.gnorm_out = gnorm_out; st.cta_sumsq = cta_sumsq; st.counter = counter4; st.tick = tick; st.seq_ptr = nullptr;
-    st.max_norm = max_grad_norm; st.lr = lr; st.b1 = b1; st.b2 = b2; st.eps = eps;
-    if (b200rl_comm_world(ctx) > 1) {   // sharded run: needs the attached peer exchange and one rank per device
-        if (!b200rl_comm_p2p_table(ctx, &st.tab) || !st.tab.exclusive || (size_t)np + 4 > kP2PXCap) return B200RL_ERR_UNSUPPORTED;
-        st.seq_ptr = b200rl_comm_p2p_seq_dev(ctx);
-    }
-    int rc = nn_tc_ac_loss_grad(ctx, 2 * ctas, actor, critic, params, hp, b, partial, loss_partial, np, &st);
-    return rc != B200RL_OK ? rc : nn_tc_partial_rows(2 * ctas, actor, hp, b.B);
+    TRY(nn_tc_ac_loss_grad(ctx, tc_grid(ctx), actor, critic, st.params, hp, b, partial, loss_partial, np, &st));
+    return nn_tc_partial_rows(tc_grid(ctx), actor, hp, b.B);
 }
 
 int nn_reduce_partials(b200rl_ctx* ctx, const float* partial, int n_partials, int64_t np, float* grad, const float* loss_partial,
@@ -1152,21 +1120,14 @@ int nn_clip_adam(b200rl_ctx* ctx, float* params, float* grad, float* m, float* v
     return B200RL_OK;
 }
 
-int nn_reduce_clip_adam(b200rl_ctx* ctx, const float* partial, int n_partials, int64_t np, float* params, float* grad, float* m, float* v,
-                        float* beta_t, const float* loss_partial, int n_loss, float* loss_out4, float max_grad_norm, float lr, float b1, float b2,
-                        float eps, float* gnorm_out, double* cta_sumsq, unsigned int* counter2, float* stats_row, unsigned int* tick) {
+int nn_reduce_clip_adam(b200rl_ctx* ctx, const float* partial, int n_partials, int64_t np, const float* loss_partial, int n_loss, const OptStep& st) {
     unsigned grid = grid_for(np, 256);
     REQUIRE((int)grid <= ctx->sm_count, B200RL_ERR_UNSUPPORTED, "fused reduce+Adam needs all CTAs co-resident");
-    P2PTable tab = {};
-    if (b200rl_comm_p2p_table(ctx, &tab)) {
+    if (st.tab.nranks > 1) {
         REQUIRE((size_t)np + 4 <= kP2PXCap, B200RL_ERR_UNSUPPORTED, "gradient larger than the peer exchange inbox");
-        reduce_clip_adam_kernel<true><<<grid, 256, 0, ctx->stream>>>(partial, n_partials, np, params, grad, m, v, beta_t, loss_partial, n_loss, loss_out4,
-                                                                    max_grad_norm, lr, b1, b2, eps, gnorm_out, cta_sumsq, counter2, stats_row, tab,
-                                                                    b200rl_comm_p2p_seq_dev(ctx), tick);
+        reduce_clip_adam_kernel<true><<<grid, 256, 0, ctx->stream>>>(partial, n_partials, np, loss_partial, n_loss, st);
     } else {
-        reduce_clip_adam_kernel<false><<<grid, 256, 0, ctx->stream>>>(partial, n_partials, np, params, grad, m, v, beta_t, loss_partial, n_loss, loss_out4,
-                                                                     max_grad_norm, lr, b1, b2, eps, gnorm_out, cta_sumsq, counter2, stats_row, tab,
-                                                                     nullptr, tick);
+        reduce_clip_adam_kernel<false><<<grid, 256, 0, ctx->stream>>>(partial, n_partials, np, loss_partial, n_loss, st);
     }
     LAUNCH_CHECK(ctx);
     return B200RL_OK;

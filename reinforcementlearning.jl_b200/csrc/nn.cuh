@@ -41,10 +41,9 @@ struct AcBatch {
     const float* norm2;         // device {mean, inv_std} for advantage normalisation
 };
 
-// Optimiser step fused into the tail of the tensor-core K7 (nn_ac_loss_grad_step): reduce the per-CTA partials -> [NVLink peer
-// exchange] -> global norm -> clip_by_global_norm! -> Adam, behind two grid barriers inside the SAME launch (the 148 persistent
-// CTAs are co-resident), instead of a second kernel (~14-20 us of launch, L2 round trips and barrier per optimiser step).
-struct AcStep {
+// Optimiser state and hyper-parameters of one optimiser step (reduce the per-CTA partials -> [NVLink peer exchange] -> global norm ->
+// clip_by_global_norm! -> Adam), whichever kernels run it (opt_path.h).
+struct OptStep {
     float* params; float* grad; float* m; float* v; float* beta_t;
     float* loss_out4; float* stats_row; float* gnorm_out;     // each may be null
     double* cta_sumsq;            // >= 148 doubles
@@ -52,15 +51,13 @@ struct AcStep {
     unsigned int* tick;           // may be null: device update counter incremented once by the launch
     unsigned int* seq_ptr;        // gradient-exchange sequence number (sharded run)
     float max_norm, lr, b1, b2, eps;
-    P2PTable tab;                 // nranks <= 1: single GPU
+    P2PTable tab;                 // nranks <= 1: no peer exchange
 };
-// K7 + optimiser step in one launch.  Returns the number of gradient partials (> 0) like nn_ac_loss_grad, or
-// B200RL_ERR_UNSUPPORTED *without side effects* when the configuration is outside the fused path (the caller then runs
-// nn_ac_loss_grad + nn_reduce_clip_adam).
-int nn_ac_loss_grad_step(b200rl_ctx* ctx, const MlpDesc& actor, const MlpDesc& critic, float* params, const AcHyper& hp, const AcBatch& b,
-                         float* partial, float* loss_partial, float* grad, float* m, float* v, float* beta_t, float* loss_out4,
-                         float max_grad_norm, float lr, float b1, float b2, float eps, float* gnorm_out, double* cta_sumsq,
-                         unsigned int* counter4, float* stats_row, unsigned int* tick);
+// K7 + optimiser step in ONE launch (OPT_FUSED_TAIL): the step runs in the tail of the tensor-core K7 behind two grid barriers (the
+// 148 persistent CTAs are co-resident) instead of a second kernel (~14-20 us of launch, L2 round trips and barrier per optimiser
+// step).  Returns the number of gradient partials (> 0) like nn_ac_loss_grad, or a negative status.
+int nn_ac_loss_grad_step(b200rl_ctx* ctx, const MlpDesc& actor, const MlpDesc& critic, const AcHyper& hp, const AcBatch& b, float* partial,
+                         float* loss_partial, const OptStep& st);
 
 #ifdef __CUDACC__
 __device__ __forceinline__ uint32_t ac_perm_key(const AcBatch& b) { return b.perm_key + (b.perm_epoch ? *b.perm_epoch * 1000003u : 0u); }
@@ -76,17 +73,17 @@ int nn_mlp_forward(b200rl_ctx* ctx, const MlpDesc& net, const float* params, con
 // Returns the number of gradient partials written (> 0; loss rows = 2x that) or a negative status.
 int nn_ac_loss_grad(b200rl_ctx* ctx, const MlpDesc& actor, const MlpDesc& critic, const float* params, const AcHyper& hp,
                     const AcBatch& b, float* partial /* [ctas][np] */, float* loss_partial /* [2*ctas][4] */);
+int nn_ac_partial_rows(b200rl_ctx* ctx, const MlpDesc& actor, const MlpDesc& critic, const AcHyper& hp, int64_t B);   // what nn_ac_loss_grad returns
+bool nn_fused_step_enabled();   // B200RL_FUSED_STEP / b200rl_set_fused_step
+bool nn_tc_fused_tail_fits(b200rl_ctx* ctx, const MlpDesc& actor, const AcHyper& hp, int64_t B, int64_t np);   // opt_fused_tail_fits for K7
 int nn_reduce_partials(b200rl_ctx* ctx, const float* partial, int n_partials, int64_t np, float* grad, const float* loss_partial,
                        int n_loss_partials, float* loss_out4);
 // clip_by_global_norm! + Optimisers Adam on a flat gradient (single CTA, deterministic)
 int nn_clip_adam(b200rl_ctx* ctx, float* params, float* grad, float* m, float* v, float* beta_t /* device [2] */, int64_t np,
                  float max_grad_norm, float lr, float b1, float b2, float eps, float grad_scale, float* gnorm_out /* device */);
-// fused single-launch variant (single GPU, or a sharded run with the NVLink peer exchange attached; stats_row (may be null)
-// receives {4 loss sums, grad norm}): cta_sumsq >= 148 doubles, counter2 = 2 zero-initialised uints (self-resetting grid barrier),
-// tick (may be null) = device counter incremented once by the launch (the agent's update counter that keys the permutation)
-int nn_reduce_clip_adam(b200rl_ctx* ctx, const float* partial, int n_partials, int64_t np, float* params, float* grad, float* m, float* v,
-                        float* beta_t, const float* loss_partial, int n_loss, float* loss_out4, float max_grad_norm, float lr, float b1, float b2,
-                        float eps, float* gnorm_out, double* cta_sumsq, unsigned int* counter2, float* stats_row, unsigned int* tick);
+// fused single-launch variant (OPT_ONE_KERNEL, OPT_ONE_KERNEL_XCHG when st.tab has peers; st.stats_row receives {4 loss sums,
+// grad norm}): needs all ceil(np / 256) CTAs co-resident
+int nn_reduce_clip_adam(b200rl_ctx* ctx, const float* partial, int n_partials, int64_t np, const float* loss_partial, int n_loss, const OptStep& st);
 int nn_target_sync(b200rl_ctx* ctx, float* target, const float* model, int64_t np, float rho);
 // DQN: TD loss + backward on a gathered batch (device arrays s (in,B), a, r, t, s2, w)
 int nn_dqn_loss_grad(b200rl_ctx* ctx, const MlpDesc& q, const float* params, const float* target, const float* s, const int32_t* a,
@@ -112,4 +109,4 @@ int nn_tc_rollout(b200rl_ctx* ctx, b200rl_env* env, const MlpDesc& actor, const 
 bool nn_tc_bwd_supported(const MlpDesc& actor, const MlpDesc& critic);
 int nn_tc_partial_rows(int grid, const MlpDesc& actor, const AcHyper& hp, int64_t B);   // gradient-partial rows the tensor-core K7 writes with `grid` CTAs
 int nn_tc_ac_loss_grad(b200rl_ctx* ctx, int grid, const MlpDesc& actor, const MlpDesc& critic, const float* params, const AcHyper& hp,
-                       const AcBatch& b, float* partial, float* loss_partial, int64_t np, const AcStep* step /* null: loss + backward only */);
+                       const AcBatch& b, float* partial, float* loss_partial, int64_t np, const OptStep* step /* null: loss + backward only */);

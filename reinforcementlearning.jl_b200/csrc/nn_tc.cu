@@ -12,7 +12,8 @@
 // must stay below 65504 in magnitude (scale 1), weights below 1023 (scale 64); gradients are scaled by ~1/(4 inv_B) at launch.
 // Below 6e-5 the lo part is subnormal: absolute error <= 2^-25 per element, far inside the 1e-5 bar.  Layer 1 (K <= 4) and the
 // heads (N <= 2) stay on FFMA.  The forward-only kernels (policy inference, fused rollout) live in fwd_tc.cu (same split).
-#include "nn.cuh"
+#include "opt_path.h"
+#include "optim.cuh"
 #include "perm.cuh"
 #include "tc_split.h"
 #include "umma.cuh"
@@ -277,7 +278,7 @@ template <int ACT>
 __global__ void __launch_bounds__(NT7_ALL, 1)
 ac_loss_grad_tc_kernel(MlpDesc actor, MlpDesc critic, const float* params /* no __restrict__: the fused optimiser step rewrites them in the tail */, AcHyper hp, AcBatch b, float* partial,
                        float* __restrict__ loss_partial, int64_t np_total, float scale_base /* power of two ~ 1 / inv_B */,
-                       AcStep st /* st.params != null: the optimiser step runs in the tail of this launch */,
+                       OptStep st /* st.params != null: the optimiser step runs in the tail of this launch */,
                        int n_actor /* CTAs [0, n_actor) work on the actor, the rest on the critic */) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     SmemBwd& sm = *reinterpret_cast<SmemBwd*>(smem_raw);
@@ -833,14 +834,7 @@ ac_loss_grad_tc_kernel(MlpDesc actor, MlpDesc critic, const float* params /* no 
         K7_T(24);                                // (everything since the last tile: drain, head-gradient reductions, partial rows)
         worker_sync();                           // every worker's partial / loss rows are written (CTA scope) ...
         K7_T(25);
-        if (tid == 0) {                          // grid barrier A: every CTA's rows are written
-            __threadfence();                     // ... and ordered before the arrival device-wide (fence cumulativity, as in cooperative groups)
-            atomicAdd(st.counter, 1u);
-            unsigned int spins = 0;
-            while (*reinterpret_cast<volatile unsigned int*>(st.counter) < G)
-                if (++spins > (1u << 26)) __trap();
-            __threadfence();
-        }
+        if (tid == 0) grid_arrive_wait(st.counter, G);   // grid barrier A: every CTA's rows are written and ordered device-wide
         worker_sync();
         K7_T(26);
         const int per = (int)((np_total + G - 1) / G);           // parameters per CTA (<= 512: checked by the launcher)
@@ -905,6 +899,7 @@ ac_loss_grad_tc_kernel(MlpDesc actor, MlpDesc critic, const float* params /* no 
             const unsigned slot = seq & 1u;
             if (mine) p2p_push(st.tab, 0, slot, (size_t)k, __float_as_uint(gk), seq);
             if (loss_thread) p2p_push(st.tab, 0, slot, (size_t)np_total + tid, __float_as_uint(lsum), seq);
+            // (rank-order sums as p2p_sum_rank_order, gradient and loss words in one loop: kept as it was, like the Adam step below)
             float acc = 0.f, lacc = 0.f;
             for (int r = 0; r < st.tab.nranks; ++r) {
                 if (mine) acc += r == st.tab.rank ? gk : __uint_as_float(p2p_recv(st.tab, 0, slot, r, (size_t)k, seq));
@@ -927,12 +922,7 @@ ac_loss_grad_tc_kernel(MlpDesc actor, MlpDesc critic, const float* params /* no 
                 double t = 0.0;
                 for (int w = 0; w < NT7 / 32; ++w) t += sm.RedD[w];
                 st.cta_sumsq[blockIdx.x] = t;
-                __threadfence();
-                atomicAdd(st.counter + 1, 1u);
-                unsigned int spins = 0;
-                while (*reinterpret_cast<volatile unsigned int*>(st.counter + 1) < G)
-                    if (++spins > (1u << 26)) __trap();
-                __threadfence();
+                grid_arrive_wait(st.counter + 1, G);
             }
             __syncwarp();
             K7_T(29);
@@ -948,9 +938,7 @@ ac_loss_grad_tc_kernel(MlpDesc actor, MlpDesc critic, const float* params /* no 
             for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
             if (lane == 0) {
                 const float gn = (float)sqrt(tot);
-                float sc = 1.0f;
-                if (st.max_norm > 0.f && st.max_norm <= gn) sc = st.max_norm / fmaxf(st.max_norm, gn);
-                sm.step_scale = sc;
+                sm.step_scale = clip_scale(gn, st.max_norm);
                 if (blockIdx.x == 0) {
                     if (st.gnorm_out) *st.gnorm_out = gn;
                     if (st.stats_row) st.stats_row[4] = gn;
@@ -963,21 +951,15 @@ ac_loss_grad_tc_kernel(MlpDesc actor, MlpDesc critic, const float* params /* no 
         if (mine) {
             gk *= sm.step_scale;
             st.grad[k] = gk;
+            // (adam_apply's arithmetic written out: through the helper, register allocation in K7's main loop changes and K7 runs ~0.7 % slower)
             const float mk = st.b1 * m_k + (1.0f - st.b1) * gk;
             const float vk = st.b2 * v_k + (1.0f - st.b2) * (gk * gk);
             st.m[k] = mk; st.v[k] = vk;
             st.params[k] = p_k - mk / (1.0f - bt1) / (sqrtf(vk / (1.0f - bt2)) + st.eps) * st.lr;
         }
         worker_sync();
-        if (tid == 0) {                          // the last CTA through advances beta^t and re-arms the counters (every thread of
-                                                 // every CTA has read beta^t / the sequence number before its CTA arrives here)
-            if (atomicAdd(st.counter + 2, 1u) + 1u == G) {
-                st.beta_t[0] = bt1 * st.b1; st.beta_t[1] = bt2 * st.b2;
-                st.counter[0] = 0u; st.counter[1] = 0u; st.counter[2] = 0u;
-                if (st.tab.nranks > 1) *st.seq_ptr = seq;
-                if (st.tick) *st.tick += 1u;
-            }
-        }
+        if (tid == 0) last_cta_epilogue(st, st.counter + 2, 3, G, bt1, bt2, st.tab.nranks > 1, seq);   // (every thread of every CTA
+                                                                                                        //  has read beta^t / seq)
         K7_T(31);
     }
     }  // worker warps
@@ -1004,14 +986,12 @@ bool nn_tc_bwd_supported(const MlpDesc& actor, const MlpDesc& critic) {
     return actor.H == 64 && critic.H == 64 && actor.in <= kInMax && actor.nout <= 2 && critic.nout == 1;
 }
 int nn_tc_ac_loss_grad(b200rl_ctx* ctx, int grid, const MlpDesc& actor, const MlpDesc& critic, const float* params, const AcHyper& hp,
-                       const AcBatch& b, float* partial, float* loss_partial, int64_t np, const AcStep* step) {
-    AcStep st = {};
+                       const AcBatch& b, float* partial, float* loss_partial, int64_t np, const OptStep* step) {
+    OptStep st = {};
     const int n_actor = nn_tc_actor_ctas(grid, actor, hp, (b.B + TM - 1) / TM);
-    if (step) {
+    if (step) {   // (opt_path chose OPT_FUSED_TAIL for these sizes)
         st = *step;
-        const int64_t per = (np + grid - 1) / grid;
-        const int rows = n_actor > grid - n_actor ? n_actor : grid - n_actor;
-        REQUIRE(st.params == params && per <= NT7 && grid <= ctx->sm_count && per * rows <= 10 * NT7 && 4 * grid <= 2 * NT7 && grid <= 256, B200RL_ERR_UNSUPPORTED,
+        REQUIRE(st.params == params && opt_fused_tail_fits(np, grid, max(n_actor, grid - n_actor), ctx->sm_count), B200RL_ERR_UNSUPPORTED,
                 "fused optimiser step: bad configuration");
     }
     size_t smem = sizeof(SmemBwd) + 128;

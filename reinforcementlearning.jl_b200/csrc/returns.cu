@@ -13,7 +13,7 @@
 //            memory with coalesced loads along time, then scans from shared memory.
 // The fused variant also emits returns = adv + v and per-CTA partial sums for the advantage
 // normalisation used by the PPO update (no second pass over the advantages).
-#include "common.cuh"
+#include "internal.h"
 #include "jl_device.cuh"
 
 namespace {

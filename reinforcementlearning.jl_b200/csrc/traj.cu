@@ -18,7 +18,7 @@
 // the episode-start frame), which reproduces the reference's entry count and sampleable set exactly.
 // A push is one thread per lane (neighbouring lanes write neighbouring addresses unless their episode counts differ);
 // a sample is one thread per batch slot: Xoshiro draw -> (rejection | sum-tree descent) -> 2 x state gather + scalars.
-#include "common.cuh"
+#include "internal.h"
 
 namespace {
 
@@ -545,7 +545,6 @@ int b200rl_traj_total_priority(b200rl_traj* t, float* out) {
 }  // extern "C"
 
 // ---- internal accessors for algo.cu -----------------------------------------------------------
-struct TrajBatchView { const float* s; const int32_t* a; const float* r; const uint8_t* t; const float* s2; const float* w; int64_t B; int ns; };
 TrajBatchView b200rl_traj_internal_batch(b200rl_traj* t) {
     return TrajBatchView{t->batch.s, t->batch.a, t->batch.r, t->batch.t, t->batch.s2, t->prioritized ? t->batch.w : nullptr, t->B, t->r.ns};
 }

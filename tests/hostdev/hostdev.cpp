@@ -1,11 +1,12 @@
 // tests/hostdev/hostdev.cpp — TEST INFRASTRUCTURE.  The product's device headers compiled for the host (see cuda_runtime.h here) behind
-// a flat C interface: Julia math kernels, Xoshiro samplers, env reset!/_step! per env, and the minibatch permutation.  The control flow
+// a flat C interface: Julia math kernels, Xoshiro samplers, env reset!/_step! per env, the minibatch permutation and the optimiser-step rule.  The control flow
 // around the per-env primitives (auto-reset after a terminating step) restates env.cu's step kernel in the obvious serial way.
 #include <cuda_runtime.h>
 
 #include <vector>
 
 #include "env_device.cuh"
+#include "opt_path.h"
 #include "perm.cuh"
 #include "tc_split.h"
 
@@ -20,6 +21,11 @@ double hd_cos64(double x) { return jld::jcos(x); }
 double hd_mod64(double x, double y) { return jld::jmod(x, y); }
 uint32_t hd_perm_index(uint32_t q, uint32_t n, uint32_t key) { return b200perm::perm_index(q, n, key); }
 int hd_tc_actor_ctas(int grid, int gaussian, int64_t ntiles) { return b200rl_tc_actor_ctas(grid, gaussian != 0, ntiles); }
+// opt_path() with the fused tail's size limits evaluated by opt_fused_tail_fits(np, grid, rows, sm_count)
+int hd_opt_path(int world, int p2p, int exclusive, int fused_step, int tc_bwd, int64_t np, int grid, int rows, int sm_count, int fits_inbox, int coresident) {
+    return opt_path(OptPathIn{world, p2p != 0, exclusive != 0, fused_step != 0, tc_bwd != 0, opt_fused_tail_fits(np, grid, rows, sm_count), fits_inbox != 0,
+                              coresident != 0});
+}
 int64_t hd_rand_oneto(uint64_t* s, uint64_t n) {
     jld::Xo g{s[0], s[1], s[2], s[3]};
     long long r = jld::rand_oneto(g, n);

@@ -5,6 +5,7 @@ and csrc/perm.cuh (minibatch permutation) are plain C++ once the CUDA qualifiers
 g++ -ffp-contract=off keeps the rounding points of the nvcc -fmad=false build.  Bit-exact agreement here means an edit of the device
 math is caught by the CPU suite; the `-m gpu` tests then only have to pin the kernels' plumbing."""
 import ctypes as C
+import itertools
 import os
 import subprocess
 
@@ -21,7 +22,7 @@ SO = os.path.join(HD, "libhostdev.so")
 
 @pytest.fixture(scope="module")
 def hd():
-    srcs = [os.path.join(HD, "hostdev.cpp"), os.path.join(HD, "cuda_runtime.h")] + [os.path.join(CSRC, f) for f in ("jl_device.cuh", "env_device.cuh", "perm.cuh", "tc_split.h")]
+    srcs = [os.path.join(HD, "hostdev.cpp"), os.path.join(HD, "cuda_runtime.h")] + [os.path.join(CSRC, f) for f in ("jl_device.cuh", "env_device.cuh", "perm.cuh", "tc_split.h", "opt_path.h")]
     if not os.path.exists(SO) or any(os.path.getmtime(s) > os.path.getmtime(SO) for s in srcs):
         cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
         subprocess.check_call([cxx, "-O2", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-mfma", "-Wno-unknown-pragmas",
@@ -29,7 +30,8 @@ def hd():
     L = C.CDLL(SO)
     vp, i32, i64, u64, f32, f64 = C.c_void_p, C.c_int, C.c_int64, C.c_uint64, C.c_float, C.c_double
     for name, res, args in (("hd_sin32", f32, [f32]), ("hd_cos32", f32, [f32]), ("hd_sin64", f64, [f64]), ("hd_cos64", f64, [f64]),
-                            ("hd_mod64", f64, [f64, f64]), ("hd_perm_index", C.c_uint32, [C.c_uint32] * 3), ("hd_tc_actor_ctas", i32, [i32, i32, i64]), ("hd_rand_oneto", i64, [vp, u64]),
+                            ("hd_mod64", f64, [f64, f64]), ("hd_perm_index", C.c_uint32, [C.c_uint32] * 3), ("hd_tc_actor_ctas", i32, [i32, i32, i64]),
+                            ("hd_opt_path", i32, [i32] * 5 + [i64] + [i32] * 5), ("hd_rand_oneto", i64, [vp, u64]),
                             ("hd_env_run", i32, [i32, vp, i64, i32, vp, vp, i32, vp, vp, vp, vp, vp, i32])):
         fn = getattr(L, name)
         fn.restype, fn.argtypes = res, args
@@ -200,3 +202,29 @@ def test_actor_critic_cta_split_rule(hd):
                 cost = lambda a: max(math.ceil(nt / a), r * math.ceil(nt / (grid - a)))
                 cands = [a for a in range(grid // 2, min(grid // 2 + 8, grid - 1) + 1)]
                 assert cost(na) <= min(cost(a) for a in cands) + 1e-9
+
+
+FUSED_TAIL, ONE_KERNEL, ONE_KERNEL_XCHG, NCCL_CHAIN = range(4)
+
+
+def test_optimiser_step_path_rule(hd):
+    """opt_path.h: which kernels run an optimiser step, for every combination of its inputs, including the sharded NCCL rows that no
+    single-GPU test reaches.  The fused tail's size limits are pinned at the BASELINE network (9 155 parameters, 148 CTAs, <= 82
+    partial rows) and just past each limit."""
+    fits = dict(np=9155, grid=148, rows=82, sm=148)
+    misfits = [dict(fits, np=148 * 512 + 1),            # > 512 parameters per CTA
+               dict(fits, rows=83),                      # 62 x 83 staged floats > 10 x 512
+               dict(fits, grid=258, sm=258),             # more CTAs than the staged loss rows allow
+               dict(fits, sm=146)]                       # not co-resident
+    for tail_fits, shape in [(True, fits)] + [(False, m) for m in misfits]:
+        for world in (1, 2, 8):
+            for p2p in ((False,) if world == 1 else (False, True)):        # a peer exchange needs peers
+                for exclusive, fused, tc, inbox, cores in itertools.product((False, True), repeat=5):
+                    got = hd.hd_opt_path(world, p2p, exclusive, fused, tc, shape["np"], shape["grid"], shape["rows"], shape["sm"], inbox, cores)
+                    if fused and tc and tail_fits and (world == 1 or (p2p and exclusive and inbox)):
+                        want = FUSED_TAIL
+                    elif (world > 1 and not p2p) or not cores:
+                        want = NCCL_CHAIN       # also on one GPU when the reduce + Adam grid cannot be co-resident
+                    else:
+                        want = ONE_KERNEL_XCHG if p2p else ONE_KERNEL   # (a gradient too large for the inbox is refused by the launcher)
+                    assert got == want, (world, p2p, exclusive, fused, tc, inbox, cores, shape)
